@@ -6,6 +6,7 @@ rCCA.fit(), 2 views, n=100000 rows per GPU, d=[1024,1024], k=64, c=0.1, float32 
     python bench.py --impl reference --steps 1 --warmup 0     # the reference algorithm on the host cores, FULL size
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...   # sample-sharded, one all-reduce
     python bench.py --workload mcca4|ccaloss64|ccaloss512     # the other BASELINE configs (same JSON contract)
+    python bench.py ... --dump-outputs DIR   # also write the last timed step's results as DIR/<name>.npy
 
 One "step" = one fit (rcca, mcca4) or one forward+backward of the objective (ccaloss*).  Under N ranks every rank
 holds its own row shard (weak scaling): the job is ONE fit over N x rows per step and its throughput is reported in
@@ -49,6 +50,18 @@ WORKLOADS = {
 }
 W = dict(WORKLOADS["rcca"])
 CPU_BUDGET_S = 150.0   # wall-clock budget of a CPU arm (the first fit always completes)
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Write what the timed path handed back in its last step as <out_dir>/<name>.npy (float32 / float64).  The inputs
+    are seeded, so two builds run with the same arguments can be compared output for output."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"outputs of {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte dump limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 class gpu_local_cpus:
@@ -384,12 +397,14 @@ def run_ours(args):
         zs = [h.to(dev).requires_grad_(True) for h in host]
         fn = CCALoss(eps=1e-5)
         flush = torch.empty(160 << 20, dtype=torch.uint8, device=dev)   # > 126 MB L2
+        last = {}
 
         def step_dev():
             flush.zero_()                       # L2 flush between timed iterations (the batch itself is 2-16 MB)
             for z in zs:
                 z.grad = None
-            fn(zs).backward()
+            last["loss"] = fn(zs)
+            last["loss"].backward()
 
         grads_host = [torch.empty_like(h).pin_memory() for h in host]
         loss_host = torch.empty((), dtype=torch.float32).pin_memory()
@@ -423,6 +438,13 @@ def run_ours(args):
     clocks = sampler.stop() if sampler else None
     lib.ccab_profile_moments(0)
     ms_per_step = total_ms / args.steps
+    if args.dump_outputs and rank == 0:   # before the end-to-end leg refits the estimator
+        if est is not None:
+            outputs = {**{f"weights_{i}": w.copy() for i, w in enumerate(est.weights_)},
+                       **{f"means_{i}": m.copy() for i, m in enumerate(est.means_)}}
+        else:
+            outputs = {"loss": last["loss"].detach().cpu().numpy(),
+                       **{f"grad_{i}": z.grad.cpu().numpy() for i, z in enumerate(zs)}}
     value = world / (ms_per_step * 1e-3)
 
     # ---- end-to-end arm: pinned host inputs -> public API -> result on the host ----
@@ -507,6 +529,8 @@ def run_ours(args):
                                                 budget_s=90.0)
         if model == "rcca":
             line["parity"] = parity_vs_oracle(est, [h.numpy() for h in host])
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -525,7 +549,13 @@ def main():
     ap.add_argument("--workload", default="rcca", choices=sorted(WORKLOADS),
                     help="rcca = BASELINE configs[1] (the headline); mcca4 = configs[3] shard; ccaloss64 / "
                          "ccaloss512 = configs[2] at the two readings of its width")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the estimator's weights_ / means_ (or the loss and its "
+                                                          "gradients) of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     W.clear()
     W.update(WORKLOADS[args.workload])
     if args.impl == "reference":

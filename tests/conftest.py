@@ -11,7 +11,6 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (authoring container only)")
 
 
 def pytest_collection_modifyitems(config, items):
@@ -22,8 +21,6 @@ def pytest_collection_modifyitems(config, items):
     except Exception:  # pragma: no cover
         has_gpu = False
     skip_gpu = pytest.mark.skip(reason="no CUDA device")
-    skip_ref = pytest.mark.skip(reason="/root/reference not present")
-    has_ref = os.path.isdir("/root/reference/cca_zoo")
     # tools/run_gpu_tests_on_standin.py: the kernels are replaced by tests/fake_ops.py, so the estimator-level gpu
     # tests can check the host logic on a CPU-only machine
     if os.environ.get("CCAB_TESTS_ON_STANDIN") == "1":
@@ -31,5 +28,3 @@ def pytest_collection_modifyitems(config, items):
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(skip_gpu)
-        if "reference" in item.keywords and not has_ref:
-            item.add_marker(skip_ref)

@@ -160,3 +160,33 @@ def cfg3_check_gradient(g, ref, view_index, case, tol):
     assert e_tr < tol, f"batch projection differs: {e_tr:.2e}"
     assert e_c < tol, f"width projection differs: {e_c:.2e}"
     return max(e_rows, e_fro, e_tr, e_c)
+
+
+# ---- outputs of the live reference for the oracle, fuzz and drop-in tests (oracle/make_golden_live.py) ----
+with open(os.path.join(_DIR, "reference_live.json")) as _f:
+    META_LIVE = json.load(_f)
+with np.load(os.path.join(_DIR, "reference_live.npz")) as _z:
+    _LIVE = {k: _z[k] for k in _z.files}
+_LIVE_INDEX = json.loads(bytes(_LIVE.pop("index")))
+
+
+def live(key):
+    """One stored array (the file holds one flat array per dtype; the index gives dtype, start and shape)."""
+    dt, start, shape = _LIVE_INDEX[key]
+    return _LIVE[dt][start:start + int(np.prod(shape))].reshape(shape)
+
+
+def live_list(key):
+    out = []
+    while f"{key}/{len(out)}" in _LIVE_INDEX:
+        out.append(live(f"{key}/{len(out)}"))
+    return out
+
+
+def sha256_matches(arrays, digests):
+    """Same dtype, shape and bytes as the arrays the stored SHA-256 digests were taken of."""
+    import hashlib
+
+    got = [[str(a.dtype), list(a.shape), hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()]
+           for a in arrays]
+    return got == digests

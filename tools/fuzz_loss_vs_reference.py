@@ -7,15 +7,13 @@ through an eigendecomposition with repeated eigenvalues and its own gradient is 
 """
 import os
 import sys
-import warnings
 
-import numpy as np
 import pytest
-import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from tests import fake_ops  # noqa: E402
+from tests import fuzz_cases as F  # noqa: E402
 from oracle import refshim  # noqa: E402
 
 refshim.install()
@@ -30,49 +28,14 @@ def main():
     seed = int(args[0]) if args else 0
     trials = int(args[1]) if len(args) > 1 else 200
     show_all = "--all" in sys.argv
-    g = torch.Generator().manual_seed(seed)
-    rng = np.random.default_rng(seed)
     bad = 0
-    for _ in range(trials):
-        kind = str(rng.choice(["CCALoss", "MCCALoss", "GCCALoss"]))
-        m = 2 if kind == "CCALoss" else int(rng.integers(2, 5))
-        n = int(rng.integers(4, 200))
-        widths = [int(rng.integers(1, 80)) for _ in range(m)]
-        if kind == "GCCALoss" or rng.random() < 0.5:
-            widths = [widths[0]] * m
-        eps = float(rng.choice([1e-3, 1e-4, 1e-5]))
-        dt = torch.float64 if rng.random() < 0.7 else torch.float32
-        lat = torch.randn(n, 3, generator=g, dtype=torch.float64)
-        zs = [(lat @ torch.randn(3, w, generator=g, dtype=torch.float64) * float(rng.uniform(0, 1.5))
-               + torch.randn(n, w, generator=g, dtype=torch.float64)).to(dt) for w in widths]
-        # rank-deficient or barely determined batch covariance (smallest eigenvalue at the rounding level of float32)
-        deficient = n - 1 <= 1.25 * (sum(widths) if kind == "GCCALoss" else max(widths))
-        if deficient and not show_all:
+    for i, t in enumerate(F.loss_trials(seed, trials)):
+        if not t["determined"] and not show_all:
             continue
-        res = []
-        for lib in (ref, ours):
-            zz = [z.clone().requires_grad_(True) for z in zs]
-            try:
-                with warnings.catch_warnings():
-                    warnings.simplefilter("ignore")
-                    loss = getattr(lib, kind)(eps=eps)(zz)
-                    loss.backward()
-                res.append((loss.item(), [z.grad.double().numpy() for z in zz], loss.dtype, loss.dim()))
-            except Exception as e:  # noqa: BLE001
-                res.append(e)
-        desc = f"{kind} n={n} widths={widths} eps={eps} {dt}"
-        r, o = res
-        if isinstance(r, Exception) or isinstance(o, Exception):
-            if type(r) is not type(o):
-                bad += 1
-                print("EXCEPTION", desc, "| ref", repr(r)[:100], "| ours", repr(o)[:100])
-            continue
-        tol = 5e-3 if dt == torch.float32 else 1e-7
-        dl = abs(r[0] - o[0]) / max(abs(r[0]), 1e-300)
-        dg = max(np.abs(a - b).max() / max(np.abs(a).max(), 1e-300) for a, b in zip(r[1], o[1]))
-        if not (dl < tol and dg < 50 * tol) or r[2:] != o[2:]:
+        msg = F.loss_mismatch(F.loss_record(ref, t, i), F.loss_record(ours, t, i), t)
+        if msg:
             bad += 1
-            print(f"VALUES loss {dl:.1e} grad {dg:.1e} dtype/dim {r[2:]} {o[2:]}", desc)
+            print(msg)
     print(f"seed {seed}: {trials} trials, {bad} mismatches")
     return 1 if bad else 0
 

@@ -8,14 +8,13 @@ where the reference itself returns noise-dependent output) are reported only wit
 """
 import os
 import sys
-import warnings
 
-import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from tests import fake_ops  # noqa: E402  (before refshim: the reference has its own `tests` package)
+from tests import fuzz_cases as F  # noqa: E402
 from oracle import refshim  # noqa: E402
 
 refshim.install()
@@ -23,7 +22,6 @@ import cca_zoo.linear as ref  # noqa: E402
 
 fake_ops.install(pytest.MonkeyPatch())
 from cca_zoo_b200 import linear as ours  # noqa: E402
-from oracle import restatement as R  # noqa: E402
 
 
 def main():
@@ -32,106 +30,13 @@ def main():
     trials = int(args[1]) if len(args) > 1 else 300
     show_all = "--all" in sys.argv
     medium = "--medium" in sys.argv        # wider views, explicit solver routes (top-k route needs 4k <= width)
-    rng = np.random.default_rng(seed)
     bad = 0
-    for _ in range(trials):
-        model = str(rng.choice(["CCA", "rCCA", "PLS", "MCCA", "GCCA", "PartialCCA", "GRCCA"]))
-        m = 2 if model in ("CCA", "rCCA", "PLS") else int(rng.integers(2, 5))
-        n = int(rng.integers(6, 120))
-        dims = [int(rng.integers(1, 30)) for _ in range(m)]
-        k = int(rng.integers(1, 8))
-        if medium:
-            n = int(rng.integers(300, 700))
-            dims = [int(rng.integers(36, 110)) for _ in range(m)]
-        lat = rng.standard_normal((n, 3))
-        views = [lat @ rng.standard_normal((3, d)) * rng.uniform(0, 1.5) + rng.standard_normal((n, d))
-                 + rng.uniform(-1, 1) for d in dims]
-        dup = rng.random() < 0.15
-        if dup:
-            j = int(rng.integers(0, m))
-            views[j] = np.hstack([views[j], views[j][:, :1]])
-            dims[j] += 1
-        f32 = rng.random() < 0.25
-        if f32:
-            views = [v.astype(np.float32) for v in views]
-        kw = dict(latent_dimensions=k, center=bool(rng.random() < 0.75))
-        c = 0.0
-        if model not in ("CCA", "PLS"):
-            c = float(rng.choice([0.0, 0.0, 0.1, 0.5, 1.0])) if rng.random() < 0.7 else \
-                [float(rng.uniform(0, 1)) for _ in range(m)]
-            kw["c"] = c
-        extra = {}
-        ours_kw = {}
-        if medium and model not in ("CCA", "PLS"):
-            ours_kw["solver"] = str(rng.choice(["auto", "eigen", "cholesky"]))
-        if model == "GCCA" and rng.random() < 0.5:
-            kw["view_weights"] = [float(rng.uniform(0.5, 2)) for _ in range(m)]
-        if model == "MCCA":
-            kw["pca"] = bool(rng.random() < 0.5)
-        if model == "PartialCCA":
-            extra["partials"] = rng.standard_normal((n, int(rng.integers(1, 4)))) + 0.3
-        if model == "GRCCA":
-            kw["mu"] = float(rng.choice([0.0, 0.5, 2.0]))
-            extra["feature_groups"] = [rng.integers(0, 3, size=d) for d in dims]
-        cmin = 1.0 if model == "PLS" else (min(c) if isinstance(c, list) else c)
-        q = extra["partials"].shape[1] if "partials" in extra else 0
-        determined = (not dup) and n - 2 - q > sum(dims)     # else exact correlation-1 ties (degenerate top eigenspace)
-        # c = 0 needs full-rank blocks; GCCA takes pinv(view) whatever c is; float32 inputs of an under-determined
-        # problem amplify the reference's own float32 rounding (centring and pinv run in float32 there)
-        well = determined or (cmin > 0 and model != "GCCA" and not f32)
-        desc = f"{'well ' if well else 'ILL  '}{model} n={n} dims={dims} f32={f32} {kw} {ours_kw}"
-        out = []
-        for lib in (ref, ours):
-            try:
-                with warnings.catch_warnings():
-                    warnings.simplefilter("ignore")
-                    est = getattr(lib, model)(**kw, **(ours_kw if lib is ours else {})).fit(views, **extra)
-                    held = [v[: n // 2] for v in views]
-                    out.append((est, est.score(views), est.transform(held), est.pairwise_correlations(held)))
-            except Exception as e:  # noqa: BLE001
-                out.append(e)
-        r, o = out
-        if isinstance(r, Exception) or isinstance(o, Exception):
-            if type(r) is not type(o):
-                bad += 1
-                print("EXCEPTION", desc, "| ref:", repr(r)[:120], "| ours:", repr(o)[:120])
-            continue
-        if not well and not show_all:
-            continue
-        if [w.shape for w in r[0].weights_] != [w.shape for w in o[0].weights_]:
+    for t in F.linear_trials(seed, trials, medium):
+        msg = F.linear_mismatch(F.linear_reduce(F.linear_record(ref, t), t), F.linear_record(ours, t, ours=True), t,
+                                show_all)
+        if msg:
             bad += 1
-            print("WEIGHT SHAPES", desc, [w.shape for w in r[0].weights_], [w.shape for w in o[0].weights_])
-            continue
-        dt_r = [w.dtype for w in r[0].weights_] + [np.asarray(t).dtype for t in r[2]]
-        dt_o = [w.dtype for w in o[0].weights_] + [np.asarray(t).dtype for t in o[2]]
-        if dt_r != dt_o:
-            bad += 1
-            print("DTYPES", desc, dt_r, dt_o)
-            continue
-        tol = 2e-3 if f32 else 1e-6
-        kmax = min(min(dims), max(n - 2 - q, 0))
-        d_score = float(np.max(np.abs(r[1] - o[1])[np.arange(r[1].shape[0]) < max(kmax, 1)])) if True else 0.0
-        # weights / variates only for components that are determined: inside the rank of the problem, clearly
-        # correlated, and separated from both neighbours (sign-aligned per component)
-        sc = r[1]
-        kmax = min(min(dims), max(n - 2 - q, 0))
-        left = np.abs(np.diff(np.concatenate([[2.0], sc])))
-        right = np.abs(np.diff(np.concatenate([sc, [-2.0]])))
-        simple = (left > 1e-3) & (right > 1e-3) & (np.abs(sc) > 1e-3) & (np.arange(sc.shape[0]) < kmax)
-        w_r = [np.asarray(w, dtype=np.float64) for w in r[0].weights_]
-        w_o = R.align_signs([np.asarray(w, dtype=np.float64) for w in o[0].weights_], w_r)
-        d_w = 0.0
-        for a, b in zip(w_o, w_r):
-            num = np.linalg.norm(a - b, axis=0)[simple]
-            den = np.linalg.norm(b, axis=0)[simple]
-            if num.size:
-                d_w = max(d_w, float(np.max(num / np.maximum(den, 1e-300))))
-        d_means = max(float(np.max(np.abs(np.asarray(a, dtype=np.float64) - np.asarray(b, dtype=np.float64))))
-                      for a, b in zip(r[0].means_, o[0].means_))
-        d_pair = float(np.max(np.abs(r[3][..., simple] - o[3][..., simple]))) if simple.any() else 0.0
-        if not (d_score < tol and d_w < 50 * tol and d_means < 1e-5 and d_pair < 50 * tol):
-            bad += 1
-            print(f"VALUES score {d_score:.1e} weights {d_w:.1e} means {d_means:.1e} pairwise {d_pair:.1e}", desc)
+            print(msg)
     print(f"seed {seed}: {trials} trials, {bad} mismatches")
     return 1 if bad else 0
 
